@@ -43,7 +43,12 @@ def parse():
     ap.add_argument("--no-lpips", action="store_true", help="reconstruction loss = L1 only")
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"],
                     help="run the step as one captured CUDA graph (auto = on)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 class ClockSampler:
@@ -173,6 +178,39 @@ def cpu_config1(reps: int = 3):
     return {"workload": "VTP-Small f16d64, batch=4 256x256, encode->decode reconstruction only, fp32, no_grad, CPU",
             "value": 4 / med, "unit": "images/sec", "ms_per_call": med * 1e3, "cores": cores, "kind": "port", "reps": reps,
             "gflop_per_image": encode_decode_flops(cfg) / 1e9}
+
+
+DUMP_SAMPLE = 1 << 21       # elements per sampled array: 2 x 8 MiB of float32
+
+
+def _canonical_sample(store, names, k: int, seed: int = 0):
+    """Indices into the flat buffers of `store` of k elements drawn with a fixed seed from the parameters `names`,
+    flattened one after the other in sorted-name order: the sample picks the same parameter elements whatever order and
+    alignment the store lays them out in."""
+    import torch
+
+    names = sorted(names)
+    sizes = torch.tensor([store.f32(n).numel() for n in names])
+    offsets = torch.tensor([store.offset[n] for n in names])
+    ends = sizes.cumsum(0)
+    pos = torch.randint(int(ends[-1]), (k,), generator=torch.Generator().manual_seed(seed)).sort().values
+    which = torch.searchsorted(ends, pos, right=True)
+    return (offsets[which] + pos - (ends[which] - sizes[which])).to(store.p.device)
+
+
+def dump_outputs(out_dir: str, tr, loss):
+    """What a caller of the training step receives from the last timed step, as float32 .npy files: `loss` (the loss
+    vector the step returns) and seeded samples (DUMP_SAMPLE elements each, see _canonical_sample) of the updated student
+    parameters (`params`) and of the updated EMA teacher (`teacher`)."""
+    import numpy as np
+
+    st = tr.store
+    os.makedirs(out_dir, exist_ok=True)
+    idx = _canonical_sample(st, st.offset, DUMP_SAMPLE)
+    tidx = _canonical_sample(st, [name for name, _, _, teacher in st.specs if teacher], DUMP_SAMPLE)
+    arrays = {"loss": loss, "params": st.p[idx], "teacher": st.tp[tidx]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def workload_config(args, world: int, flops_per_image: float, image_groups=None) -> dict:
@@ -325,6 +363,9 @@ def main():
     ms_e2e = max_over_ranks(e2.elapsed_time(e3))
     log(f"end-to-end: {ms_e2e / args.steps:.1f} ms/step")
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr, loss_host)
+        log(f"outputs of the last step written to {args.dump_outputs}")
     # ---- dominant kernel: the tcgen05 GEMM (gemm_kernel<256,4,NONE>), timed live on its largest recurring shape on the
     #      hot path: the FFN fc1 projection of the SSL student pass (bias, bf16 out; the SwiGLU gate is a separate pass)
     Mg, Ng, Kg = 2 * B * 257, 2 * tr.hs, tr.D

@@ -30,3 +30,31 @@ def test_reference_arm_prints_one_contract_line():
     args = argparse.Namespace(batch=256, model="small", prototypes=65536, no_lpips=False)
     ours = bench.workload_config(args, 1, d["config"]["flops_per_image"])
     assert {k: d["config"][k] for k in ours} == ours and "sample" in d["config"]
+
+
+def test_dump_sample_follows_parameters_not_store_layout():
+    """`bench.py --dump-outputs` samples the same parameter elements whatever order and padding the flat parameter store
+    gives them, so that two builds can be compared output for output."""
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+    from vtp_b200.train import ParamStore
+
+    def store(specs):
+        st = ParamStore("cpu")
+        for name, shape in specs:
+            st.add(name, shape)
+        st.finalize()
+        for name in st.offset:
+            v = st.f32(name)
+            v.copy_(torch.arange(v.numel()).view_as(v) + 1000.0 * ord(name))
+        return st
+
+    specs = [("a", (3, 5)), ("b", (7,)), ("c", (4, 4))]
+    s1, s2 = store(specs), store(specs[::-1])
+    assert s1.offset != s2.offset
+    i1, i2 = (bench._canonical_sample(s, s.offset, 500) for s in (s1, s2))
+    assert torch.equal(s1.p[i1], s2.p[i2])
+    assert (s1.p[i1] >= 1000.0 * ord("a")).all()                  # never the zero padding between parameters
+    assert set(s1.p[i1].div(1000, rounding_mode="floor").long().tolist()) == {ord("a"), ord("b"), ord("c")}

@@ -1,70 +1,49 @@
 """Caption tokenizer (vtp_b200/text_tokenizer.py, SURVEY.md §8(f)4) — CPU tests.
 
-  * against the LIVE reference `SimpleTokenizer` (vtp/tokenizers/text_tokenizer.py:144-295) with the reference's own
-    vocabulary file: identical vocabulary, identical ids for every caption of a corpus built to hit the pattern's
-    branches, identical truncation and decoding.  Runs only where /root/reference exists (the dev container); the
-    vocabulary is the reference's data file and is not committed;
+  * against the reference `SimpleTokenizer` (vtp/tokenizers/text_tokenizer.py:144-295), recorded by
+    oracle/make_golden_tokenizer.py on a corpus built to hit the pattern's branches: identical vocabulary, identical ids
+    for every caption, identical truncation and decoding.  The vocabulary is the reference's data file reduced to the
+    merges that corpus uses (tests/golden/tokenizer_bpe.txt.gz; the reduction leaves every caption's split unchanged);
   * self-contained cases on a tiny synthetic vocabulary (written to a temp dir): merge order, end-of-word variants,
     special tokens, truncation rule, errors."""
 import gzip
-import importlib.util
 import os
-import random
 
 import pytest
 import torch
 
+from oracle.make_golden_tokenizer import EXTRA, LENGTHS, VOCAB, corpus, digest
+from tests.util import load_golden
 from vtp_b200.text_tokenizer import BPETokenizer, find_bpe_file, get_tokenizer
 
-REF_TOK = "/root/reference/vtp/tokenizers/text_tokenizer.py"
-REF_BPE = "/root/reference/tools/bpe_simple_vocab_16e6.txt.gz"
 
-CORPUS = [
-    "a photo of a cat", "A Photo of a CAT!!!", "  multiple   spaces\tand\nnewlines ",
-    "it's the dog's ball, they've won; I'm here, we'll go, he'd say, don't", "'s't're've'm'll'd", "''''",
-    "naïve café déjà vu — “quotes” ‘single’ … ellipsis", "日本語のテキスト と 中文文本 and한국어", "emoji 😀😃 🤖👍🏽 flags 🇩🇪",
-    "numbers 1234567890 3.14159 1e-5 ½ ²", "&amp;lt;b&amp;gt; html &amp; entities &lt;i&gt; &#39;x&#39;",
-    "<start_of_text> literal specials <end_of_text> inside", "<START_OF_TEXT> upper special", "", "   ", "x", "a" * 300,
-    "word " * 200, "supercalifragilisticexpialidocious antidisestablishmentarianism",
-    "e-mail: someone@example.com, http://example.com/path?query=1&b=2", "tabs\tand\x00control\x07chars",
-    "mixed123abc456 under_score-dash", "ÀÉÎÕÜ ßẞ ǅ İi", "𝔘𝔫𝔦𝔠𝔬𝔡𝔢 math 𝟘𝟙𝟚", "！？。、", "á combining ë",
-]
-
-
-def _load_reference_tokenizer():
-    spec = importlib.util.spec_from_file_location("_ref_text_tokenizer", REF_TOK)   # by path: `import vtp` needs omegaconf
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
-
-
-@pytest.mark.skipif(not (os.path.exists(REF_TOK) and os.path.exists(REF_BPE)), reason="needs the reference checkout")
 def test_token_ids_equal_the_live_reference():
-    ref_mod = _load_reference_tokenizer()
-    ours, ref = BPETokenizer(REF_BPE), ref_mod.SimpleTokenizer(REF_BPE)
-    assert ours.encoder == ref.encoder and ours.decoder == ref.decoder and ours.byte_decoder == ref.byte_decoder
-    assert (ours.vocab_size, ours.sot_token_id, ours.eot_token_id, ours.all_special_ids, ours.context_length) == \
-           (ref.vocab_size, ref.sot_token_id, ref.eot_token_id, ref.all_special_ids, ref.context_length)
-    rng = random.Random(0)
-    alphabet = "abcdefghijklmnopqrstuvwxyz  ABC.,!?'0123456789-éüñ日本😀"
-    corpus = CORPUS + ["".join(rng.choice(alphabet) for _ in range(rng.randint(1, 120))) for _ in range(400)]
-    for text in corpus:
-        a, b = ours.encode(text), ref.encode(text)
-        assert a == b, text
-        assert ours.decode(a) == ref.decode(b)
-    for L in (None, 8, 16, 77, 200):            # padding, exact fit, truncation (last slot becomes <end_of_text>)
-        x, y = ours(corpus, L), ref(corpus, L)
-        assert x.dtype == torch.long and torch.equal(x, y)
-    assert torch.equal(ours("one caption"), ref("one caption"))
+    meta, g = load_golden("tokenizer")
+    h = meta["sha256"]
+    texts = corpus()
+    assert digest(texts) == meta["corpus_sha256"]
+    ours = BPETokenizer(VOCAB)
+    assert digest(sorted(ours.encoder.items())) == h["encoder"] and digest(sorted(ours.decoder.items())) == h["decoder"]
+    assert digest(sorted(ours.byte_decoder.items())) == h["byte_decoder"]
+    assert [ours.vocab_size, ours.sot_token_id, ours.eot_token_id, ours.all_special_ids, ours.context_length] == \
+           [meta[k] for k in ("vocab_size", "sot_token_id", "eot_token_id", "all_special_ids", "context_length")]
+    ref_ids = torch.split(g["ids_flat"].long(), g["ids_len"].tolist())
+    ids = [ours.encode(text) for text in texts]
+    for text, a, b in zip(texts, ids, ref_ids):
+        assert a == b.tolist(), text
+    assert digest([ours.decode(a) for a in ids]) == h["decoded"]
+    for L in LENGTHS:                           # padding, exact fit, truncation (last slot becomes <end_of_text>)
+        x = ours(texts, L)
+        assert x.dtype == torch.long and digest(x.tolist()) == h[f"batch_{L}"], L
+    assert digest(ours("one caption").tolist()) == h["one_caption"]
     # second call: served from the caption cache, same ids
-    assert torch.equal(ours(corpus), ref(corpus))
+    assert digest(ours(texts).tolist()) == h["batch_None"]
     # no lower-casing + an extra special token (case-sensitive cache hit of specials, as upstream)
-    o2 = BPETokenizer(REF_BPE, clean="whitespace", additional_special_tokens=["<mask>"])
-    r2 = ref_mod.SimpleTokenizer(REF_BPE, clean="whitespace", additional_special_tokens=["<mask>"])
-    extra = corpus + ["Keep CASE <mask> <Mask> <start_of_text>"]
-    assert torch.equal(o2(extra), r2(extra)) and o2.vocab_size == r2.vocab_size == ours.vocab_size + 1
-    # the lookup finds the reference's copy when a checkout is importable, and get_tokenizer mirrors the factory
-    assert get_tokenizer(bpe_path=REF_BPE, context_length=32)("a cat").shape == (1, 32)
+    o2 = BPETokenizer(VOCAB, clean="whitespace", additional_special_tokens=["<mask>"])
+    assert digest(o2(texts + EXTRA).tolist()) == h["extra_special"]
+    assert o2.vocab_size == meta["vocab_size_extra_special"] == ours.vocab_size + 1
+    # get_tokenizer mirrors the factory
+    assert get_tokenizer(bpe_path=VOCAB, context_length=32)("a cat").shape == (1, 32)
 
 
 def _tiny_vocab(tmp_path):
