@@ -125,8 +125,10 @@ int vtp_l2norm_fwd(const void* x, int x_dtype, void* y, int y_dtype, float* norm
  * ------------------------------------------------------------------------------------------------------------ */
 /* layers/attention.py:110-126 after RoPE (F.scaled_dot_product_attention, scale 1/8, head_dim 64) and the causal
  * nn.MultiheadAttention of layers/block.py:387-412.  qkv bf16 [B*T][3*H*64] packed [q|k|v] x [H][64]; out bf16
- * [B*T][H*64]; lse fp32 [B][H][T] optional (saved for backward).  `prefix` leading tokens (cls) are computed on CUDA
- * cores, the other T-prefix (<=256) tokens on tcgen05. */
+ * [B*T][H*64]; lse fp32 [B][H][T] optional (saved for backward).  `prefix` (<= 4) leading tokens (cls) are computed
+ * on CUDA cores, the other HW = T-prefix tokens on tcgen05: HW <= 256 by the single-pass kernels (attention.cu,
+ * attention_pipe.cu; causal allowed), HW > 256 by the key-streaming online-softmax kernel (attention_long.cu;
+ * non-causal only, a causal call returns VTP_ERR_ARG). */
 int vtp_attention_fwd(const void* qkv, void* out, float* lse, int B, int T, int H, int prefix, int causal,
                       vtp_stream_t stream);
 /* same op on fp32 tensors (CUDA cores) for the fp32-accurate inference mode */

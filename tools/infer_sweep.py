@@ -1,6 +1,6 @@
 """Config 5 of BASELINE.json: encode+decode inference throughput sweep (bf16 autocast mode).  GPU only.  (Latents parity
 against the reference lives in tests/test_model_gpu.py — tools never touch oracle/.)
-  python tools/infer_sweep.py --model large --batches 1,8,64,256 [--graphs]
+  python tools/infer_sweep.py --model large --batches 1,8,64,256 [--graphs] [--image-size 512]
 --graphs also times CUDA-graph replays (VTPModel.enable_cuda_graphs) — the small-batch serving path."""
 import argparse
 import json
@@ -18,14 +18,15 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--model", default="large")
 ap.add_argument("--batches", default="1,8,64,256")
 ap.add_argument("--graphs", action="store_true")
+ap.add_argument("--image-size", type=int, default=256, help="square input size (256: BASELINE config 5)")
 a = ap.parse_args()
 cfg = preset(a.model)
 torch.manual_seed(0)
 m = VTPModel(cfg).cuda()
-fl = encode_decode_flops(cfg)
-out = {"model": a.model, "gflop_per_image": fl / 1e9, "rows": []}
+fl = encode_decode_flops(cfg, a.image_size)
+out = {"model": a.model, "image_size": a.image_size, "gflop_per_image": fl / 1e9, "rows": []}
 for B in [int(b) for b in a.batches.split(",")]:
-    x = torch.randn(B, 3, 256, 256, device="cuda")
+    x = torch.randn(B, 3, a.image_size, a.image_size, device="cuda")
     with torch.autocast("cuda", dtype=torch.bfloat16):
         for _ in range(3):
             rec = m.get_latents_decoded_images(m.get_reconstruction_latents(x))

@@ -11,7 +11,10 @@
 // The `prefix` (cls / storage) tokens — 1 in the encoder, 0 in the decoder/text — would cost a third 128-row tile for
 // one row, so they are handled on CUDA cores: their key columns are folded into every row's softmax by the row
 // threads, and their query rows are computed by a spare warp from the K/V tiles already in smem.
+// Sequences with more than 256 non-prefix tokens go to the key-streaming kernel of attention_long.cu.
 #include <stdlib.h>
+
+#include <algorithm>
 
 #include "attention.h"
 #include "host.h"
@@ -690,56 +693,95 @@ __global__ void __launch_bounds__(ATT8_THREADS, 2) attn_fwd8_kernel(const __grid
 namespace vtp {
 
 // ------------------------------------------------------------------------------------------------------------
-// fp32 attention (accuracy mode): CUDA cores, one CTA per (head, image), K/V tiles in padded smem, one warp per
-// query row.  Used by the fp32-exact inference mode only (layers/attention.py:124 with fp32 q,k,v).
+// fp32 attention (accuracy mode): CUDA cores, one CTA per (head, image), K/V in padded smem, one warp per query row.
+// Used by the fp32-exact inference mode only (layers/attention.py:124 with fp32 q,k,v).
+// K/V go through smem in chunks of C keys (the host picks the largest C that fits, C = T whenever the whole sequence
+// does).  Each chunk updates the row's running max / sum / accumulator; with a single chunk the first update is a plain
+// assignment, so those shapes run exactly the arithmetic of a one-pass softmax.  With several chunks the query rows go in
+// rounds of nw * F32_ROWS rows whose running state stays in registers while the chunks stream past.
+static constexpr int F32_ROWS = 8;  // query rows per warp per round
 __global__ void attn_fwd_f32_kernel(const float* __restrict__ qkv, float* __restrict__ out, int T, int H, int causal,
-                                    float scale) {
+                                    float scale, int C) {
     extern __shared__ float sm[];
     const int D = H * 64, h = blockIdx.x, b = blockIdx.y;
-    float* Ks = sm;                 // [T][65]
-    float* Vs = Ks + (long)T * 65;  // [T][64]
-    float* Ps = Vs + (long)T * 64;  // [nwarps][T]
+    float* Ks = sm;                 // [C][65]
+    float* Vs = Ks + (long)C * 65;  // [C][64]
+    float* Ps = Vs + (long)C * 64;  // [nwarps][C]
     const float* base = qkv + (long)b * T * 3 * D;
-    for (int i = threadIdx.x; i < T * 64; i += blockDim.x) {
-        const int t = i >> 6, d = i & 63;
-        Ks[t * 65 + d] = base[(long)t * 3 * D + D + h * 64 + d];
-        Vs[t * 64 + d] = base[(long)t * 3 * D + 2 * D + h * 64 + d];
+    auto load_chunk = [&](int c0) {
+        const int n = min(C, T - c0);
+        for (int i = threadIdx.x; i < n * 64; i += blockDim.x) {
+            const int t = i >> 6, d = i & 63;
+            Ks[t * 65 + d] = base[(long)(c0 + t) * 3 * D + D + h * 64 + d];
+            Vs[t * 64 + d] = base[(long)(c0 + t) * 3 * D + 2 * D + h * 64 + d];
+        }
+    };
+    const bool resident = C >= T;
+    if (resident) {
+        load_chunk(0);
+        __syncthreads();
     }
-    __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-    float* pw = Ps + (long)warp * T;
-    for (int q = warp; q < T; q += nw) {
-        const float* qp = base + (long)q * 3 * D + h * 64;
-        float qf[64];
+    float* pw = Ps + (long)warp * C;
+    for (int q0 = 0; q0 < T; q0 += nw * F32_ROWS) {
+        float m[F32_ROWS], l[F32_ROWS], a0[F32_ROWS], a1[F32_ROWS];
+        for (int c0 = 0; c0 < T; c0 += C) {
+            if (!resident) {
+                __syncthreads();  // every warp is done with the previous chunk
+                load_chunk(c0);
+                __syncthreads();
+            }
 #pragma unroll
-        for (int d = 0; d < 64; ++d) qf[d] = qp[d];
-        const int kend = causal ? q + 1 : T;
-        float m = -INFINITY;
-        for (int k = lane; k < kend; k += 32) {
-            float acc = 0.f;
+            for (int i = 0; i < F32_ROWS; ++i) {
+                const int q = q0 + warp + nw * i;
+                if (q >= T) continue;
+                const int kend = min(causal ? q + 1 : T, c0 + C) - c0;  // visible keys of this chunk
+                if (kend <= 0) continue;                                // causal: the whole chunk lies ahead of q
+                const float* qp = base + (long)q * 3 * D + h * 64;
+                float qf[64];
 #pragma unroll
-            for (int d = 0; d < 64; ++d) acc += qf[d] * Ks[k * 65 + d];
-            acc *= scale;
-            pw[k] = acc;
-            m = fmaxf(m, acc);
+                for (int d = 0; d < 64; ++d) qf[d] = qp[d];
+                float mc = -INFINITY;
+                for (int k = lane; k < kend; k += 32) {
+                    float acc = 0.f;
+#pragma unroll
+                    for (int d = 0; d < 64; ++d) acc += qf[d] * Ks[k * 65 + d];
+                    acc *= scale;
+                    pw[k] = acc;
+                    mc = fmaxf(mc, acc);
+                }
+                mc = warp_max(mc);
+                const float mn = c0 == 0 ? mc : fmaxf(m[i], mc);
+                float lc = 0.f;
+                for (int k = lane; k < kend; k += 32) {
+                    const float e = expf(pw[k] - mn);
+                    pw[k] = e;
+                    lc += e;
+                }
+                lc = warp_sum(lc);
+                __syncwarp();
+                float x0 = 0.f, x1 = 0.f;
+                for (int k = 0; k < kend; ++k) {
+                    const float pk = pw[k];
+                    x0 += pk * Vs[k * 64 + lane], x1 += pk * Vs[k * 64 + 32 + lane];
+                }
+                if (c0 == 0) {
+                    l[i] = lc, a0[i] = x0, a1[i] = x1;
+                } else {
+                    const float alpha = expf(m[i] - mn);
+                    l[i] = l[i] * alpha + lc, a0[i] = a0[i] * alpha + x0, a1[i] = a1[i] * alpha + x1;
+                }
+                m[i] = mn;
+                __syncwarp();
+            }
         }
-        m = warp_max(m);
-        float l = 0.f;
-        for (int k = lane; k < kend; k += 32) {
-            const float e = expf(pw[k] - m);
-            pw[k] = e;
-            l += e;
+#pragma unroll
+        for (int i = 0; i < F32_ROWS; ++i) {
+            const int q = q0 + warp + nw * i;
+            if (q >= T) continue;
+            float* op = out + ((long)b * T + q) * D + h * 64;
+            op[lane] = a0[i] / l[i], op[32 + lane] = a1[i] / l[i];
         }
-        l = warp_sum(l);
-        __syncwarp();
-        float a0 = 0.f, a1 = 0.f;
-        for (int k = 0; k < kend; ++k) {
-            const float pk = pw[k];
-            a0 += pk * Vs[k * 64 + lane], a1 += pk * Vs[k * 64 + 32 + lane];
-        }
-        float* op = out + ((long)b * T + q) * D + h * 64;
-        op[lane] = a0 / l, op[32 + lane] = a1 / l;
-        __syncwarp();
     }
 }
 
@@ -752,7 +794,8 @@ extern "C" int vtp_attention_fwd(const void* qkv, void* out, float* lse, int B, 
     VTP_CHECK_ARG(qkv && out && B > 0 && T > 0 && H > 0, "attention_fwd: bad args");
     VTP_CHECK_ARG(prefix >= 0 && prefix <= MAX_PREFIX && prefix < T, "attention_fwd: prefix must be in [0,%d]", MAX_PREFIX);
     const int HW = T - prefix;
-    VTP_CHECK_ARG(HW <= 256, "attention_fwd: %d non-prefix tokens > 256 is not supported by the single-pass kernel", HW);
+    VTP_CHECK_ARG(HW <= 256 || !causal,
+                  "attention_fwd: causal attention over %d non-prefix tokens (> 256) is not supported", HW);
     VTP_CHECK_ARG(B <= 65535 && H <= 65535, "attention_fwd: grid too large");
     const int D = H * 64;
     AttnDev p;
@@ -762,6 +805,8 @@ extern "C" int vtp_attention_fwd(const void* qkv, void* out, float* lse, int B, 
     p.scale = 0.125f;
     p.scale_log2 = 0.125f * 1.4426950408889634f;
     p.pack = 0;
+    // more than 256 patch tokens: the score row no longer fits TMEM -> key-block streaming kernel (attention_long.cu)
+    if (HW > 256) return attn_fwd_long_launch(p, (cudaStream_t)st);
     if (!causal && T <= 64 && B > 1 && getenv("VTP_ATTN_NO_PACK") == nullptr) {
         // several whole sequences per 128-row tile; the prefix tokens become ordinary rows / columns
         p.pack = 128 / T;
@@ -795,14 +840,16 @@ extern "C" int vtp_attention_fwd(const void* qkv, void* out, float* lse, int B, 
 extern "C" int vtp_attention_fwd_f32(const float* qkv, float* out, int B, int T, int H, int causal, vtp_stream_t st) {
     VTP_CHECK_ARG(qkv && out && B > 0 && T > 0 && H > 0 && B <= 65535, "attention_fwd_f32: bad args");
     const int nw = 8;
-    const size_t smem = ((size_t)T * 65 + (size_t)T * 64 + (size_t)nw * T) * sizeof(float);
-    VTP_CHECK_ARG(smem <= 220 * 1024, "attention_fwd_f32: T=%d too long for the smem-resident kernel", T);
+    // K/V chunk: the whole sequence when it fits in 220 KB of smem, otherwise the largest chunk that does
+    const size_t per_key = (65 + 64 + nw) * sizeof(float);
+    const int C = (int)std::min<size_t>((size_t)T, 220 * 1024 / per_key);
+    const size_t smem = (size_t)C * per_key;
     static size_t configured = 0;
     if (smem > configured) {
         VTP_CUDA(cudaFuncSetAttribute(attn_fwd_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         configured = smem;
     }
-    attn_fwd_f32_kernel<<<dim3(H, B), nw * 32, smem, (cudaStream_t)st>>>(qkv, out, T, H, causal, 0.125f);
+    attn_fwd_f32_kernel<<<dim3(H, B), nw * 32, smem, (cudaStream_t)st>>>(qkv, out, T, H, causal, 0.125f, C);
     VTP_LAUNCH_CHECK();
     return VTP_OK;
 }

@@ -20,5 +20,7 @@ struct AttnDev {
 
 // persistent ping-pong forward for 128 < HW <= 256 (attention_pipe.cu); default for those shapes, VTP_ATTN_FWD_PIPE=0 opts out
 int attn_fwd_pipe_launch(const CUtensorMap& tm, const AttnDev& p, cudaStream_t st);
+// flash-style forward for HW > 256, non-causal (attention_long.cu); builds its own per-image [B][T][3D] tensor map
+int attn_fwd_long_launch(const AttnDev& p, cudaStream_t st);
 
 }  // namespace vtp

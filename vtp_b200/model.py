@@ -395,9 +395,6 @@ class VTPModel(VTPPreTrainedModel):
         ps = self.config.vision_patch_size
         if image.shape[-1] % ps or image.shape[-2] % ps:
             raise ValueError(f"image size {tuple(image.shape[-2:])} is not a multiple of the patch size {ps}")
-        if (image.shape[-1] // ps) * (image.shape[-2] // ps) > 256 and self._mode() == "bf16":
-            raise NotImplementedError(f"image {tuple(image.shape[-2:])}: more than 256 patch tokens per image; the bf16 "
-                                      "attention kernels are single-pass over <= 256 keys (+cls) — see INTEGRATION.md")
         if not image.is_cuda:
             raise lib.VtpError("VTPModel inputs must live on the CUDA device (no CPU path)")
 
